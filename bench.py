@@ -8,8 +8,11 @@ Workload (one "step"): YOLOv4-608, 3 FPN scales x 3 anchors, 80 classes, batch 1
 per GPU of synthetic head outputs + labels:
     fused CIoU loss forward+gradient (all scales, one launch)
     -> decode at joint-confidence 0.5 -> per-class DIoU-NMS at 0.45.
-`value`  : images/s, inputs resident in HBM, timed with CUDA events (max over ranks); the step
-           is two launches over static buffers replayed from a CUDA graph (--no-graph: eager).
+`value`  : images/s over exactly --steps steps, inputs resident in HBM, timed with CUDA events (max
+           over ranks); the step is two launches over static buffers replayed from a CUDA graph
+           (--no-graph: eager).
+`--dump-outputs DIR`: after the timed steps, what the last one returned (see dump_outputs) as
+           DIR/<name>.npy; the inputs are seeded, so two builds can be compared output for output.
 `e2e`    : same step through the reference-facing Python API with HOST buffers
            (pinned H2D of labels + head outputs inside the timed region, D2H of the
            loss scalars and the NMS survivors; the gradient stays on the device for
@@ -20,6 +23,7 @@ per GPU of synthetic head outputs + labels:
            bounded sample of the same workload.  TensorFlow is not installable here.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -36,7 +40,7 @@ METRIC = "images/sec YOLOv4-608 loss+grad+decode+NMS"
 UNIT = "images/s"
 CONFIG_NAME = "v4-608"
 IMG_SIZE = (608, 608)
-MIN_TIMED_S = 0.5
+DUMP_SAMPLE = 1 << 21                # gradient elements per scale that --dump-outputs keeps (8 MB each)
 # both arms print this string (the driver compares the arms' configs)
 WORKLOAD = ("YOLOv4-608 (BASELINE configs[2]): 3 scales (19/38/76) x 3 anchors, 80 classes, batch 128 per GPU; "
             "CIoU loss fwd+grad + decode(thr 0.5) + per-class DIoU-NMS(thr 0.45)")
@@ -89,6 +93,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", f"--id={self.gpu}", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                  "-lms", "20"], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)     # the sampler never outlives the benchmark, however it ends
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except Exception:
@@ -228,6 +233,27 @@ def h2d_ceiling(host_tensors, dev_tensors, barrier, reps=4):
     e1.record()
     barrier()
     return nbytes * reps / (e0.elapsed_time(e1) * 1e-3) / 1e9
+
+
+def dump_outputs(out_dir, loss, dpreds, res):
+    """Write what one step returned to its caller as out_dir/<name>.npy (at most 33 MB in all):
+    loss.npy          float32 [n_scales], the loss per scale
+    dpred<s>.npy      float32, DUMP_SAMPLE elements of scale s's gradient at the flat indices
+                      np.sort(np.random.default_rng(s).choice(numel, DUMP_SAMPLE, replace=False))
+    out_rows.npy      float64 [kept, 7], the NMS survivors of all images
+    out_offsets.npy   float64 [n_img + 1], where each image's survivors start in out_rows"""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n_kept = int(res["out_offsets"][-1].item())
+    arrays = {"loss": loss.cpu().numpy().astype(np.float32),
+              "out_rows": res["out_rows"][:n_kept].cpu().numpy().astype(np.float64),
+              "out_offsets": res["out_offsets"].cpu().numpy().astype(np.float64)}
+    for si, d in enumerate(dpreds):
+        flat = d.reshape(-1)
+        idx = np.random.default_rng(si).choice(flat.numel(), min(DUMP_SAMPLE, flat.numel()), replace=False)
+        arrays[f"dpred{si}"] = flat[torch.from_numpy(np.sort(idx)).to(flat.device)].cpu().numpy().astype(np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_ours(args):
@@ -394,38 +420,31 @@ def run_ours(args):
         clocks.wait_first_sample(lambda: (fused_losses(fns, dev_t, dev_p, global_batch=global_batch, dpreds=dpreds),
                                           torch.cuda.synchronize()))
     barrier()
-    # the timed region: rounds of exactly `steps` steps, repeated until >= MIN_TIMED_S have been
-    # measured; ms_per_step is the MEDIAN round (every rank runs the same number of rounds)
-    round_ms = []
+    # the timed region: exactly `steps` steps (every rank runs the same number)
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_begin = time.perf_counter()
-    n_rounds = 1
+    ev0.record()
+    if static_steps is not None:
+        for k in range(args.steps):
+            g_out = static_step(k)
+        out = (g_out[0], None, g_out[3])
+    else:
+        for _ in range(args.steps):
+            out = step(dev_t, dev_p, record=True)
+    join_collectives()              # the timed steps end when every step's collective has completed
+    ev1.record()
+    barrier()
+    ms = agree(ev0.elapsed_time(ev1), dist.ReduceOp.MAX if world > 1 else None) / args.steps
+    if args.dump_outputs and rank == 0:     # before anything else writes the gradient buffers
+        dump_outputs(args.dump_outputs, out[0], dpreds, out[2])
     eager_rounds = 0
-    while len(round_ms) < n_rounds:
-        barrier()
-        ev0.record()
-        if static_steps is not None:
-            for k in range(args.steps):
-                g_out = static_step(k)
-            out = (g_out[0], None, g_out[3])
-        else:
-            for _ in range(args.steps):
-                out = step(dev_t, dev_p, record=True)
-        join_collectives()              # the round ends when every step's collective has completed
-        ev1.record()
-        barrier()
-        round_ms.append(agree(ev0.elapsed_time(ev1), dist.ReduceOp.MAX if world > 1 else None))
-        if len(round_ms) == 1:
-            n_rounds = int(min(200, max(1, np.ceil(MIN_TIMED_S * 1e3 / max(round_ms[0], 1e-3)))))
-        if static_steps is not None and len(round_ms) % 4 == 1:
-            # the loss kernel alone cannot be bracketed inside a graph: between the timed rounds the
-            # same step runs as two eager launches with an event between them (not counted in ms)
-            for _ in range(args.steps):
-                eager_out = step(dev_t, dev_p, record=True)
-            join_collectives()
-            eager_rounds += 1
-    t_end = time.perf_counter()
-    ms = float(np.median(round_ms)) / args.steps
+    if static_steps is not None:
+        # the loss kernel alone cannot be bracketed inside a graph: after the timed steps the same
+        # step runs as two eager launches with an event between them (not counted in ms)
+        for _ in range(args.steps):
+            eager_out = step(dev_t, dev_p, record=True)
+        barrier()                       # its events are read next
+        eager_rounds = 1
     loss_ms = float(np.median([a.elapsed_time(b) for a, b in loss_ev]))
     loss_vals = out[0].cpu().numpy().tolist()
     if static_steps is not None:   # the replayed step returns what the eager step returned
@@ -456,23 +475,16 @@ def run_ours(args):
     kept_ref = out[2]["out_rows"][:kept_rows].cpu().numpy()
     if not np.array_equal(np.concatenate([r for r, _ in res["rows"]], axis=0), kept_ref):
         raise SystemExit("e2e survivors differ from the device-resident step's")
-    e2e_steps = max(3, min(args.steps, 10))
-    e2e_round_ms, e2e_wall_ms = [], []
-    n_rounds = 1
-    while len(e2e_round_ms) < n_rounds:
-        barrier()
-        t0 = time.perf_counter()
-        ev0.record()
-        for _ in range(e2e_steps):
-            res = pipe.run(host_p, host_boxes, host_offs)
-        ev1.record(pipe.compute_stream)
-        barrier()
-        e2e_wall_ms.append((time.perf_counter() - t0) * 1e3)
-        e2e_round_ms.append(agree(ev0.elapsed_time(ev1), dist.ReduceOp.MAX if world > 1 else None))
-        if len(e2e_round_ms) == 1:
-            n_rounds = int(min(20, max(1, np.ceil(MIN_TIMED_S * 1e3 / max(e2e_round_ms[0], 1e-3)))))
+    barrier()
+    t0 = time.perf_counter()
+    ev0.record()
+    for _ in range(args.steps):
+        res = pipe.run(host_p, host_boxes, host_offs)
+    ev1.record(pipe.compute_stream)
+    barrier()
+    e2e_wall_ms = (time.perf_counter() - t0) * 1e3 / args.steps
+    e2e_ms = agree(ev0.elapsed_time(ev1), dist.ReduceOp.MAX if world > 1 else None) / args.steps
     t_end = time.perf_counter()
-    e2e_ms = float(np.median(e2e_round_ms)) / e2e_steps
     clock_info = clocks.stop(t_begin, t_end) if rank == 0 else None   # samples inside both timed regions
     ceiling = agree(h2d_ceiling(host_p, pipe.y_pred, barrier), dist.ReduceOp.MIN if world > 1 else None)
 
@@ -491,13 +503,12 @@ def run_ours(args):
                                     "counting pass riding on its read of y_pred, then decode + NMS with one CTA per "
                                     "image; roofline counts only the loss's algorithmic bytes"
                                     % ("_clean, replayed from a CUDA graph by engine.TrainEvalStep; the loss kernel's "
-                                       "own duration is taken from eager rounds of the same step run between the "
-                                       "timed rounds" if static_steps is not None else ""),
+                                       "own duration is taken from the same steps run eagerly after the timed "
+                                       "ones" if static_steps is not None else ""),
                            "chain": "7 launches per step: loss fwd+grad + decode counting pass (yb_loss_decode_fused), "
                                     "scan, emit, NMS classify / scatter / sweep / emit",
                            "unfused": "separate loss and decode launches"}[mode],
-                "timing": f"median of {len(round_ms)} rounds of {args.steps} steps (CUDA events, max over ranks, "
-                          f">= {MIN_TIMED_S} s measured)",
+                "timing": f"{args.steps} steps (CUDA events, max over ranks)",
                 "l2_policy": f"inputs larger than L2: {sum(a.numel() * 4 for a in dev_p + dev_t) / 1e6:.0f} MB read + "
                              f"{sum(d.numel() * 4 for d in dpreds) / 1e6:.0f} MB written per step vs 126 MB L2",
                 "decode_rows_per_image": total_rows / batch, "nms_kept_per_image": kept_rows / batch,
@@ -508,17 +519,17 @@ def run_ours(args):
             "clocks": clock_info,
             "e2e": {"value": global_batch / (e2e_ms * 1e-3), "unit": UNIT, "h2d_bytes_per_step": h2d,
                     "d2h_bytes_per_step": pipe.d2h_bytes(res["n_rows"]), "ms_per_step": e2e_ms,
-                    "wall_ms_per_step": float(np.median(e2e_wall_ms)) / e2e_steps,
+                    "wall_ms_per_step": e2e_wall_ms,
                     "h2d_gbs": h2d / (e2e_ms * 1e-3) / 1e9, "h2d_ceiling_gbs": ceiling,
                     "frac_of_h2d_ceiling": (h2d / (e2e_ms * 1e-3) / 1e9) / ceiling,
-                    "chunks": len(pipe.chunks), "rounds": len(e2e_round_ms), "steps_per_round": e2e_steps,
+                    "chunks": len(pipe.chunks), "steps": args.steps,
                     "note": "HostBatchStep: pinned head outputs + box lists in (labels encoded on the device), "
                             "loss scalars + NMS survivors written to mapped host memory; H2D of chunk k+1 under the "
                             "kernels of chunk k, one host sync per step; gradient stays on the device. "
                             "h2d_ceiling_gbs = the same head outputs copied with plain pinned cudaMemcpyAsync, "
                             "all ranks at once, nothing else running"},
-            "gpu_launches": LAUNCHES_PER_STEP[mode] * args.steps * (len(round_ms) + eager_rounds)
-                            + pipe.launches_per_step * e2e_steps * len(e2e_round_ms),
+            "gpu_launches": LAUNCHES_PER_STEP[mode] * args.steps * (1 + eager_rounds)
+                            + pipe.launches_per_step * args.steps,
             "gpu_launches_per_step": LAUNCHES_PER_STEP[mode],
             "roofline": {"bound": "hbm",
                          "kernel": "loss_fwd_bwd_kernel<4,false,%s>" % ("false" if args.unfused else "true"),
@@ -586,7 +597,13 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --batch images per GPU (default); strong: --batch images in total, split over the GPUs")
     ap.add_argument("--chunks", type=int, default=8, help="image chunks of the pipelined end-to-end step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA arm's outputs (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

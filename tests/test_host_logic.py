@@ -87,8 +87,13 @@ def test_error_behaviour_matches_the_reference():
         tools.soft_nms(np.zeros(0))
     with pytest.raises(YoloB200Error):
         km.kmeans(np.random.rand(10, 2), 2, lambda a, b: a, 1e-3)     # arbitrary Python distance
-    with pytest.raises(YoloB200Error):
-        km.iou_dist(np.ones((1, 1, 2)), np.ones((1, 1 << 17, 2)))      # data-sized host call refused
+    centre, data = np.array([[[0.3, 0.5]]]), np.random.default_rng(0).uniform(0.1, 1.0, (1, 1 << 17, 2))
+    if torch.cuda.is_available():      # a data-sized call runs on the device and gives the host formula
+        ca, da = 0.3 * 0.5, data[..., 0] * data[..., 1]
+        assert np.allclose(km.iou_dist(centre, data), 1 - np.minimum(ca, da) / np.maximum(ca, da), rtol=0, atol=1e-12)
+    else:                              # without a device it is refused, not run on the host
+        with pytest.raises(YoloB200Error):
+            km.iou_dist(centre, data)
     c = np.array([[[0.2, 0.4]], [[0.5, 0.5]]])
     assert np.allclose(km.iou_dist(c, c), 0) and np.allclose(km.euclidean_dist(c, c), 0)
     assert km.iou(c[0], c[1])[0] == (0.2 * 0.4) / (0.5 * 0.5)

@@ -21,13 +21,6 @@
 
 namespace yb {
 
-template <typename T>
-__device__ __forceinline__ T mul_rn(T a, T b);
-template <>
-__device__ __forceinline__ float mul_rn<float>(float a, float b) { return __fmul_rn(a, b); }
-template <>
-__device__ __forceinline__ double mul_rn<double>(double a, double b) { return __dmul_rn(a, b); }
-
 // K1: persistent CTAs; a producer warp streams tiles of cells through a shared-memory
 // ring with 1-D bulk-async copies (TMA), consumer warps own whole cells (lane = cell*B + box),
 // each lane walks the C class scores of its box (lanes are an odd number of words apart ->
@@ -37,8 +30,7 @@ constexpr int kDecStages = 3;
 
 template <typename T, bool kBuckets>
 __global__ void __launch_bounds__((kDecMaxConsumerWarps + 1) * 32)
-decode_count_kernel(const __grid_constant__ DecodeLaunch L, unsigned int* __restrict__ counts,
-                    unsigned int* __restrict__ n_hot, HotBox* __restrict__ hot_boxes, const HotBuckets K) {
+decode_count_kernel(const __grid_constant__ DecodeLaunch L, const __grid_constant__ DecodeSink K) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ uint64_t full[kDecStages], done[kDecStages];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -104,67 +96,16 @@ decode_count_kernel(const __grid_constant__ DecodeLaunch L, unsigned int* __rest
             for (int c0 = warp * cpw; c0 < nc; c0 += ncw * cpw) {
                 const int cell = c0 + lc;
                 const bool valid = lane_on && cell < nc;
-                int n = 0;
-                if (valid) {
-                    const T* box = sp + (size_t)cell * pcf + lb * ((L.version == 1) ? 5 : 5 + C);
-                    const T* prob = (L.version == 1) ? sp + (size_t)cell * pcf + 5 * B : box + 5;
-                    const T c = box[4];
-#pragma unroll 16
-                    for (int k = 0; k < C; ++k) n += (mul_rn<T>(c, prob[k]) >= thr) ? 1 : 0;
-                }
-                int tot = 0, before = 0;
-                for (int q = 0; q < B; ++q) {
-                    const int nq = __shfl_sync(0xffffffffu, n, lc * B + q);
-                    tot += nq;
-                    before += (q < lb) ? nq : 0;
-                }
-                unsigned my_img = 0, my_cellpos = 0, my_cis = 0;
-                if (valid) {
-                    const long long g = cell0 + cell;
-                    const long long img = g / L.cells[s];
-                    const long long o = img * L.cell_base[L.n_scales] + L.cell_base[s] + (g - img * L.cells[s]);
-                    if (lb == 0 && counts != nullptr) counts[o] = (unsigned)tot;
-                    if (n > 0 && hot_boxes != nullptr)
-                        hot_boxes[atomicAdd(n_hot, 1u)] = make_hot(o, (unsigned)g, s, lb, (unsigned)before);
-                    my_img = (unsigned)img;
-                    my_cellpos = (unsigned)(o - img * L.cell_base[L.n_scales]);
-                    my_cis = ((unsigned)s << 28) | (unsigned)(g - img * L.cells[s]);
-                }
+                const int box_at = cell * pcf + lb * ((L.version == 1) ? 5 : 5 + C);
+                const int prob_at = (L.version == 1) ? cell * pcf + 5 * B : box_at + 5;
+                const T c = valid ? sp[box_at + 4] : (T)0;
+                const LaneHits h = decode_count_lane<T>(K, valid, sp + prob_at, c, thr, C, B, lc, lb, s, cell0 + cell);
                 if (kBuckets) {
-                    // rows of the boxes with hits into their image's bucket, the warp serving one hot
-                    // box at a time (see the fused loss kernel)
-                    unsigned hot = __ballot_sync(0xffffffffu, valid && n > 0);
-                    unsigned my_base = 0;   // every hot lane reserves its rows first: the round trips overlap
-                    if (valid && n > 0) my_base = atomicAdd(&K.n[my_img], (unsigned)n);
-                    while (hot) {
-                        const int src = __ffs(hot) - 1;
-                        hot &= hot - 1;
-                        const int hcell = __shfl_sync(0xffffffffu, cell, src), hlb = __shfl_sync(0xffffffffu, lb, src);
-                        const unsigned himg = __shfl_sync(0xffffffffu, my_img, src);
-                        const unsigned hpos = __shfl_sync(0xffffffffu, my_cellpos, src);
-                        const unsigned hcis = __shfl_sync(0xffffffffu, my_cis, src);
-                        unsigned u = __shfl_sync(0xffffffffu, my_base, src);
-                        const T* hbox = sp + (size_t)hcell * pcf + hlb * ((L.version == 1) ? 5 : 5 + C);
-                        const T* hprob = (L.version == 1) ? sp + (size_t)hcell * pcf + 5 * B : hbox + 5;
-                        const T hc = hbox[4];
-                        FusedRow* dst = K.row + (size_t)himg * K.cap;
-                        for (int k0 = 0; k0 < C; k0 += 32) {
-                            const int k = k0 + lane;
-                            const T p = (k < C) ? hprob[k] : (T)0;
-                            const bool hit = (k < C) && (mul_rn<T>(hc, p) >= thr);
-                            const unsigned m = __ballot_sync(0xffffffffu, hit);
-                            const unsigned at = u + __popc(m & ((1u << lane) - 1u));
-                            if (hit && at < (unsigned)K.cap) {
-                                FusedRow fr;
-                                fr.key = fused_key(hpos, hlb, k);
-                                fr.x = (float)hbox[0]; fr.y = (float)hbox[1]; fr.w = (float)hbox[2]; fr.h = (float)hbox[3];
-                                fr.c = (float)hc; fr.p = (float)p;
-                                fr.cell = hcis;
-                                dst[at] = fr;
-                            }
-                            u += __popc(m);
-                        }
+                    T x = 0, y = 0, w = 0, hgt = 0;
+                    if (h.n > 0) {
+                        x = sp[box_at]; y = sp[box_at + 1]; w = sp[box_at + 2]; hgt = sp[box_at + 3];
                     }
+                    decode_file_rows<T>(K.buckets, h, sp, prob_at, lb, x, y, w, hgt, c, thr, C, lane);
                 }
             }
             mbar_arrive(&done[stage]);
@@ -274,9 +215,18 @@ int decode_fill(const void* const* preds, int64_t n_img, const yb_decode_params*
     return YB_OK;
 }
 
+DecodeSink decode_sink(const DecodeLaunch& L, unsigned int* counts, unsigned int* n_hot, HotBox* hot,
+                       const HotBuckets& buckets) {
+    DecodeSink K{counts, n_hot, hot, buckets, L.cell_base[L.n_scales], {}, {}, (float)L.thr};
+    for (int s = 0; s < L.n_scales; ++s) {
+        K.cell_base[s] = L.cell_base[s];
+        K.cells[s] = L.cells[s];
+    }
+    return K;
+}
+
 // K1 geometry (3 stages of <= 24 KB, 3 CTAs per SM) + launch
-int decode_count(DecodeLaunch& L, bool is_f64, unsigned int* counts, unsigned int* n_hot, HotBox* hot,
-                 const HotBuckets& buckets, cudaStream_t stream) {
+int decode_count(DecodeLaunch& L, bool is_f64, const DecodeSink& K, cudaStream_t stream) {
     const size_t esz = is_f64 ? 8 : 4;
     const int stage_budget = 24 * 1024;
     int ncw = 1, stage_bytes = 0;
@@ -300,18 +250,18 @@ int decode_count(DecodeLaunch& L, bool is_f64, unsigned int* counts, unsigned in
     const int grid = max(1, min(n_tiles, kNumSMs * ctas_per_sm));
     const int threads1 = (ncw + 1) * 32;
     if (is_f64) {
-        if (buckets.n != nullptr) return YB_E_PARAM;   // row buckets hold the float32 head values
+        if (K.buckets.n != nullptr) return YB_E_PARAM;   // row buckets hold the float32 head values
         static SmemRaised done;
         YB_CUDA_TRY(raise_dynamic_smem_once(decode_count_kernel<double, false>, (int)smem, &done));
-        decode_count_kernel<double, false><<<grid, threads1, smem, stream>>>(L, counts, n_hot, hot, buckets);
-    } else if (buckets.n != nullptr) {
+        decode_count_kernel<double, false><<<grid, threads1, smem, stream>>>(L, K);
+    } else if (K.buckets.n != nullptr) {
         static SmemRaised done;
         YB_CUDA_TRY(raise_dynamic_smem_once(decode_count_kernel<float, true>, (int)smem, &done));
-        decode_count_kernel<float, true><<<grid, threads1, smem, stream>>>(L, counts, n_hot, hot, buckets);
+        decode_count_kernel<float, true><<<grid, threads1, smem, stream>>>(L, K);
     } else {
         static SmemRaised done;
         YB_CUDA_TRY(raise_dynamic_smem_once(decode_count_kernel<float, false>, (int)smem, &done));
-        decode_count_kernel<float, false><<<grid, threads1, smem, stream>>>(L, counts, n_hot, hot, buckets);
+        decode_count_kernel<float, false><<<grid, threads1, smem, stream>>>(L, K);
     }
     YB_CUDA_TRY(cudaGetLastError());
     return YB_OK;
@@ -404,7 +354,7 @@ extern "C" int yb_decode(const void* const* preds, int64_t n_img, const yb_decod
         return YB_OK;
     }
     YB_CUDA_TRY(cudaMemsetAsync(ws.n_hot, 0, ws.zero_bytes, stream));
-    rc = decode_count(L, p->is_f64 != 0, ws.counts, ws.n_hot, ws.hot, HotBuckets{}, stream);
+    rc = decode_count(L, p->is_f64 != 0, decode_sink(L, ws.counts, ws.n_hot, ws.hot, HotBuckets{}), stream);
     if (rc != YB_OK) return rc;
     return decode_finish(L, ws, p->is_f64 != 0, rows, row_capacity, reinterpret_cast<long long*>(row_offsets), stream, true);
 }

@@ -551,9 +551,9 @@ static int fused_launch(const DecodeLaunch& D, const FusedWs& W, int row_cap, do
     return YB_OK;
 }
 
-// Shared with loss.cu (yb_loss_decode_nms_fused): workspace carve-up + memset, then the launch.
-int fused_prepare(const void* const* preds, int64_t n_img, const yb_decode_params* p, int row_cap, void* workspace,
-                  size_t workspace_bytes, DecodeLaunch& D, HotBuckets& K, cudaStream_t stream, bool clear) {
+// validation + workspace carve-up (no launches)
+static int fused_setup(const void* const* preds, int64_t n_img, const yb_decode_params* p, int row_cap,
+                       void* workspace, size_t workspace_bytes, DecodeLaunch& D, FusedWs& W) {
     int rc = fused_check(p, n_img, row_cap);
     if (rc != YB_OK) return rc;
     rc = decode_fill(preds, n_img, p, D);
@@ -563,8 +563,16 @@ int fused_prepare(const void* const* preds, int64_t n_img, const yb_decode_param
         return YB_E_WORKSPACE;
     for (int s = 0; s < D.n_scales; ++s)
         if (D.n_img * D.cells[s] > 0xffffffffll || D.B[s] > 32) return YB_E_SHAPE;
-    FusedWs W;
     fused_layout(n_img, row_cap, &W, reinterpret_cast<char*>(workspace));
+    return YB_OK;
+}
+
+// Shared with loss.cu (yb_loss_decode_nms_fused): fused_setup + memset, then the launch.
+int fused_prepare(const void* const* preds, int64_t n_img, const yb_decode_params* p, int row_cap, void* workspace,
+                  size_t workspace_bytes, DecodeLaunch& D, HotBuckets& K, cudaStream_t stream, bool clear) {
+    FusedWs W;
+    const int rc = fused_setup(preds, n_img, p, row_cap, workspace, workspace_bytes, D, W);
+    if (rc != YB_OK) return rc;
     if (clear) YB_CUDA_TRY(cudaMemsetAsync(W.zero, 0, W.zero_bytes, stream));
     K = W.K;
     return YB_OK;
@@ -608,7 +616,7 @@ extern "C" int yb_decode_nms(const void* const* preds, int64_t n_img, const yb_d
     HotBuckets K;
     int rc = fused_prepare(preds, n_img, p, rows_per_img_cap, workspace, workspace_bytes, D, K, stream);
     if (rc != YB_OK) return rc;
-    rc = decode_count(D, false, nullptr, nullptr, nullptr, K, stream);
+    rc = decode_count(D, false, decode_sink(D, nullptr, nullptr, nullptr, K), stream);
     if (rc != YB_OK) return rc;
     return fused_finish(D, n_img, rows_per_img_cap, workspace, nms_threshold, iou_mode, out_rows, out_capacity,
                         out_offsets, n_overflow, stream);
@@ -625,14 +633,10 @@ extern "C" int yb_decode_nms_finish(const void* const* preds, int64_t n_img, con
     if (out_rows == nullptr && out_capacity > 0) return YB_E_NULL;
     if (out_capacity < 0) return YB_E_CAPACITY;
     if (iou_mode != 1 && iou_mode != 2) return YB_E_PARAM;
-    int rc = fused_check(p, n_img, rows_per_img_cap);
-    if (rc != YB_OK) return rc;
-    if (workspace_bytes < fused_layout(n_img, rows_per_img_cap, nullptr, nullptr) || ((uintptr_t)workspace & 255))
-        return YB_E_WORKSPACE;
     DecodeLaunch D;
-    rc = decode_fill(preds, n_img, p, D);
-    if (rc != YB_OK) return rc;
-    if (n_img == 0) return YB_OK;
-    return fused_finish(D, n_img, rows_per_img_cap, workspace, nms_threshold, iou_mode, out_rows, out_capacity,
-                        out_offsets, n_overflow, stream);
+    FusedWs W;
+    const int rc = fused_setup(preds, n_img, p, rows_per_img_cap, workspace, workspace_bytes, D, W);
+    if (rc != YB_OK || n_img == 0) return rc;
+    return fused_launch(D, W, rows_per_img_cap, nms_threshold, iou_mode, out_rows, out_capacity,
+                        reinterpret_cast<long long*>(out_offsets), n_overflow, stream);
 }

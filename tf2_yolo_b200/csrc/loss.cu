@@ -95,16 +95,7 @@ struct LossLaunch {
     double* terms_out;     // [n_scales][YB_LOSS_TERMS] or null
     double* metrics_out;   // [n_scales][YB_LOSS_METRICS] or null
     int from_logits;       // all scales: y_pred holds raw head outputs
-    // fused decode counting (yb_loss_decode_fused): per-cell hit counts in decode OUTPUT order
-    int dec_on;                              // select the counting variant of the kernel
-    unsigned int* dec_counts;                // may be null (per-image buckets only)
-    unsigned int* dec_n_hot;
-    HotBox* dec_hot;                         // may be null
-    HotBuckets dec_buckets;                  // per-image lists for the fused decode+NMS kernel, or off
-    long long dec_per_img;                   // cells per image over all scales
-    long long dec_cell_base[YB_MAX_SCALES];  // first cell of a scale inside an image
-    long long dec_cells[YB_MAX_SCALES];      // grid_h * grid_w
-    float dec_thr;
+    DecodeSink dec;        // the decode counting pass riding on the kernel (kDecode)
 };
 
 // ---- box geometry ------------------------------------------------------------
@@ -471,41 +462,15 @@ loss_fwd_bwd_kernel(const __grid_constant__ LossLaunch L) {
                     }
                 }
                 const float resp = (lb == amax) ? 1.f : 0.f;
-                int dec_n = 0;                                            // hits of this lane's box
-                unsigned my_img = 0, my_cellpos = 0, my_cis = 0, my_base = 0;
-                if (kDecode) {
-                    // head decode, counting pass (utils/tools.py:411-412), on the tile that is already in
-                    // shared memory: hits of c*p_k >= thr per cell, stored in decode OUTPUT order, cells
-                    // with hits appended to the emit work list.  Must precede the in-place gradient writes.
-                    int n = 0;
-                    if (valid) {
-                        const float* prob = (V == 1) ? sp + cell * S.pcf + 5 * B : pc + 5;
-#pragma unroll 16
-                        for (int k = 0; k < C; ++k) n += (__fmul_rn(c, prob[k]) >= L.dec_thr) ? 1 : 0;
-                    }
-                    int tot = 0, before = 0;
-                    for (int q = 0; q < B; ++q) {
-                        const int nq = __shfl_sync(0xffffffffu, n, lc * B + q);
-                        tot += nq;
-                        before += (q < lb) ? nq : 0;
-                    }
-                    dec_n = n;
-                    if (valid) {
-                        const long long g = cell0 + cell;
-                        const long long img = g / L.dec_cells[s];
-                        const long long o = img * L.dec_per_img + L.dec_cell_base[s] + (g - img * L.dec_cells[s]);
-                        if (lb == 0 && L.dec_counts != nullptr) L.dec_counts[o] = (unsigned)tot;
-                        if (n > 0 && L.dec_hot != nullptr)
-                            L.dec_hot[atomicAdd(L.dec_n_hot, 1u)] = make_hot(o, (unsigned)g, s, lb, (unsigned)before);
-                        my_img = (unsigned)img;
-                        my_cellpos = (unsigned)(o - img * L.dec_per_img);
-                        my_cis = ((unsigned)s << 28) | (unsigned)(g - img * L.dec_cells[s]);
-                    }
-                    // a hot lane reserves its rows in the image's bucket NOW and uses them after the loss
-                    // arithmetic below: the atomic's round trip to L2 hides behind it
-                    if (L.dec_buckets.n != nullptr && valid && n > 0)
-                        my_base = atomicAdd(&L.dec_buckets.n[my_img], (unsigned)n);
-                }
+                // head decode, counting pass (utils/tools.py:411-412), on the tile that is already in
+                // shared memory.  It reserves the rows of a hot box in its image's bucket NOW; they are
+                // filed after the loss arithmetic below, which hides the atomic's round trip to L2.
+                // Both must precede the in-place gradient writes.
+                const int prob_at = cell * S.pcf + ((V == 1) ? 5 * B : lb * bstride + 5);   // the box's class scores
+                LaneHits dec = {0, 0u, 0u, 0u, 0u};
+                if (kDecode)
+                    dec = decode_count_lane<float>(L.dec, valid, sp + prob_at, c, L.dec.thr, C, B, lc, lb, s,
+                                                   cell0 + cell);
                 if (kMetrics) {
                     // In-training metrics of yolov*/metrics/yolo_metrics.py folded into this pass (they
                     // read the same tensors): objectness accuracy, mean best IoU, class accuracy, recall.
@@ -655,42 +620,8 @@ loss_fwd_bwd_kernel(const __grid_constant__ LossLaunch L) {
                         g2 *= pw; g3 *= ph;
                     }
                 }
-                if (kDecode && L.dec_buckets.n != nullptr) {
-                    // rows of the boxes with hits into their image's bucket (before the gradients overwrite
-                    // the tile): the WARP serves one hot box at a time (32 class scores per step, ballot,
-                    // lane-parallel row writes) - a lane walking its own C scores again would stall the
-                    // other 31 for C steps
-                    unsigned hot = __ballot_sync(0xffffffffu, valid && dec_n > 0);
-                    while (hot) {
-                        const int src = __ffs(hot) - 1;
-                        hot &= hot - 1;
-                        const int hcell = __shfl_sync(0xffffffffu, cell, src), hlb = __shfl_sync(0xffffffffu, lb, src);
-                        const float hc = __shfl_sync(0xffffffffu, c, src);
-                        const float hx = __shfl_sync(0xffffffffu, px, src), hy = __shfl_sync(0xffffffffu, py, src);
-                        const float hw = __shfl_sync(0xffffffffu, pw, src), hh = __shfl_sync(0xffffffffu, ph, src);
-                        const unsigned himg = __shfl_sync(0xffffffffu, my_img, src);
-                        const unsigned hpos = __shfl_sync(0xffffffffu, my_cellpos, src);
-                        const unsigned hcis = __shfl_sync(0xffffffffu, my_cis, src);
-                        unsigned u = __shfl_sync(0xffffffffu, my_base, src);
-                        const float* hprob = (V == 1) ? sp + hcell * S.pcf + 5 * B : sp + hcell * S.pcf + hlb * bstride + 5;
-                        FusedRow* dst = L.dec_buckets.row + (size_t)himg * L.dec_buckets.cap;
-                        for (int k0 = 0; k0 < C; k0 += 32) {
-                            const int k = k0 + lane;
-                            const float p = (k < C) ? hprob[k] : 0.f;
-                            const bool hit = (k < C) && (__fmul_rn(hc, p) >= L.dec_thr);
-                            const unsigned m = __ballot_sync(0xffffffffu, hit);
-                            const unsigned at = u + __popc(m & ((1u << lane) - 1u));
-                            if (hit && at < (unsigned)L.dec_buckets.cap) {
-                                FusedRow fr;
-                                fr.key = fused_key(hpos, hlb, k);
-                                fr.x = hx; fr.y = hy; fr.w = hw; fr.h = hh; fr.c = hc; fr.p = p;
-                                fr.cell = hcis;
-                                dst[at] = fr;
-                            }
-                            u += __popc(m);
-                        }
-                    }
-                }
+                if (kDecode && L.dec.buckets.n != nullptr)   // before the gradients overwrite the tile
+                    decode_file_rows<float>(L.dec.buckets, dec, sp, prob_at, lb, px, py, pw, ph, c, L.dec.thr, C, lane);
                 if (valid) {
                     if (write) {
                         pc[0] = g0; pc[1] = g1; pc[2] = g2; pc[3] = g3; pc[4] = g4;
@@ -893,8 +824,8 @@ static int launch_loss_logits(const LossLaunch& L, int grid, int threads, size_t
 }
 
 template <int V>
-static int launch_loss(const LossLaunch& L, int grid, int threads, size_t smem, cudaStream_t stream) {
-    const bool m = L.metrics_out != nullptr, d = L.dec_on != 0;
+static int launch_loss(const LossLaunch& L, bool d, int grid, int threads, size_t smem, cudaStream_t stream) {
+    const bool m = L.metrics_out != nullptr;
     if (L.from_logits) {
         if (V != 3 && V != 4) return YB_E_PARAM;  // v1/v2 heads end in a softmax
         if (d) return YB_E_PARAM;                 // decode counting needs activated scores
@@ -926,14 +857,10 @@ extern "C" size_t yb_loss_workspace_bytes(int n_scales) {
     return loss_gacc_bytes(n_scales) + 256;
 }
 
-struct FusedDecode {   // optional: count decode hits inside the loss pass
-    const DecodeLaunch* L;
-    const DecodeWs* ws;
-};
-
+// dec: optional, count decode hits inside the loss pass
 static int loss_impl(const yb_loss_scale* scales, int n_scales, float* loss_out, double* terms_out,
                      double* metrics_out, double recall_iou_threshold, void* workspace,
-                     size_t workspace_bytes, yb_stream_t stream_, const FusedDecode* fd = nullptr,
+                     size_t workspace_bytes, yb_stream_t stream_, const DecodeSink* dec = nullptr,
                      bool workspace_is_clean = false) {
     cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
     if (scales == nullptr || loss_out == nullptr || workspace == nullptr) return YB_E_NULL;
@@ -1009,19 +936,7 @@ static int loss_impl(const yb_loss_scale* scales, int n_scales, float* loss_out,
     L.terms_out = terms_out;
     L.metrics_out = metrics_out;
     for (int s = 0; s < n_scales; ++s) L.sc[s].recall_thr = (float)recall_iou_threshold;
-    if (fd != nullptr) {
-        L.dec_on = 1;
-        L.dec_counts = fd->ws->counts;
-        L.dec_n_hot = fd->ws->n_hot;
-        L.dec_hot = fd->ws->hot;
-        L.dec_buckets = fd->ws->buckets;
-        L.dec_per_img = fd->L->cell_base[n_scales];
-        for (int s = 0; s < n_scales; ++s) {
-            L.dec_cell_base[s] = fd->L->cell_base[s];
-            L.dec_cells[s] = fd->L->cells[s];
-        }
-        L.dec_thr = (float)fd->L->thr;
-    }
+    if (dec != nullptr) L.dec = *dec;
 
     const size_t smem = (size_t)n_stages * stage_bytes + acc_bytes(ncw) + bar_bytes;
     const int threads = (ncw + 1) * 32;
@@ -1031,10 +946,10 @@ static int loss_impl(const yb_loss_scale* scales, int n_scales, float* loss_out,
     if (!workspace_is_clean)
         YB_CUDA_TRY(cudaMemsetAsync(workspace, 0, loss_gacc_bytes(n_scales) + kCtrlWords * sizeof(unsigned int), stream));
     switch (version) {
-        case 1: return launch_loss<1>(L, grid, threads, smem, stream);
-        case 2: return launch_loss<2>(L, grid, threads, smem, stream);
-        case 3: return launch_loss<3>(L, grid, threads, smem, stream);
-        default: return launch_loss<4>(L, grid, threads, smem, stream);
+        case 1: return launch_loss<1>(L, dec != nullptr, grid, threads, smem, stream);
+        case 2: return launch_loss<2>(L, dec != nullptr, grid, threads, smem, stream);
+        case 3: return launch_loss<3>(L, dec != nullptr, grid, threads, smem, stream);
+        default: return launch_loss<4>(L, dec != nullptr, grid, threads, smem, stream);
     }
 }
 
@@ -1052,6 +967,34 @@ extern "C" int yb_loss_fwd_bwd_metrics(const yb_loss_scale* scales, int n_scales
                      workspace_bytes, stream);
 }
 
+// The decode parameters and head pointers of the float32 heads the loss scales hold; every scale must
+// hold the same images, of one version and class count.  YB_OK / YB_E_*.
+static int loss_decode_params(const yb_loss_scale* scales, int n_scales, double threshold, yb_decode_params& dp,
+                              const void** preds, int64_t& n_img) {
+    memset(&dp, 0, sizeof(dp));
+    dp.version = scales[0].p.version;
+    dp.class_num = scales[0].p.class_num;
+    dp.n_scales = n_scales;
+    dp.is_f64 = 0;
+    dp.threshold = threshold;
+    n_img = -1;
+    for (int s = 0; s < n_scales; ++s) {
+        const yb_loss_params& p = scales[s].p;
+        if (p.grid_h <= 0 || p.grid_w <= 0) return YB_E_SHAPE;
+        const int64_t cells = (int64_t)p.grid_h * p.grid_w;
+        if (scales[s].n_cells % cells != 0) return YB_E_SHAPE;
+        const int64_t n = scales[s].n_cells / cells;
+        if (n_img >= 0 && n != n_img) return YB_E_SHAPE;
+        n_img = n;
+        if (p.class_num != dp.class_num || p.version != dp.version) return YB_E_PARAM;
+        dp.grid_h[s] = p.grid_h;
+        dp.grid_w[s] = p.grid_w;
+        dp.bbox_num[s] = p.bbox_num;
+        preds[s] = scales[s].y_pred;
+    }
+    return YB_OK;
+}
+
 // Loss fwd+grad AND head decode of the same head outputs: y_pred is read from HBM once for both.
 extern "C" int yb_loss_decode_fused(const yb_loss_scale* scales, int n_scales, float* loss_out,
                                     double* terms_out, double decode_threshold, double* rows,
@@ -1065,31 +1008,13 @@ extern "C" int yb_loss_decode_fused(const yb_loss_scale* scales, int n_scales, f
     const bool count_only = row_offsets == nullptr;  // rows are emitted later by yb_decode_finish
     if (row_capacity < 0) return YB_E_CAPACITY;
     yb_decode_params dp;
-    memset(&dp, 0, sizeof(dp));
-    dp.version = scales[0].p.version;
-    dp.class_num = scales[0].p.class_num;
-    dp.n_scales = n_scales;
-    dp.is_f64 = 0;
-    dp.threshold = decode_threshold;
     const void* preds[YB_MAX_SCALES];
-    int64_t n_img = -1;
-    for (int s = 0; s < n_scales; ++s) {
-        const yb_loss_params& p = scales[s].p;
-        if (p.grid_h <= 0 || p.grid_w <= 0) return YB_E_SHAPE;
-        const int64_t cells = (int64_t)p.grid_h * p.grid_w;
-        if (scales[s].n_cells % cells != 0) return YB_E_SHAPE;
-        const int64_t n = scales[s].n_cells / cells;
-        if (n_img >= 0 && n != n_img) return YB_E_SHAPE;  // every scale must hold the same images
-        n_img = n;
-        if (p.class_num != dp.class_num || p.version != dp.version) return YB_E_PARAM;
-        dp.grid_h[s] = p.grid_h;
-        dp.grid_w[s] = p.grid_w;
-        dp.bbox_num[s] = p.bbox_num;
-        preds[s] = scales[s].y_pred;
-    }
+    int64_t n_img;
+    int rc = loss_decode_params(scales, n_scales, decode_threshold, dp, preds, n_img);
+    if (rc != YB_OK) return rc;
     DecodeLaunch DL;
     DecodeWs ws;
-    int rc = decode_setup(preds, n_img, &dp, decode_workspace, decode_workspace_bytes, DL, ws);
+    rc = decode_setup(preds, n_img, &dp, decode_workspace, decode_workspace_bytes, DL, ws);
     if (rc != YB_OK) return rc;
     if (ws.total_cells == 0) {
         if (!count_only) YB_CUDA_TRY(cudaMemsetAsync(row_offsets, 0, sizeof(int64_t) * (n_img + 1), stream));
@@ -1097,9 +1022,9 @@ extern "C" int yb_loss_decode_fused(const yb_loss_scale* scales, int n_scales, f
                          stream_);
     }
     YB_CUDA_TRY(cudaMemsetAsync(ws.n_hot, 0, ws.zero_bytes, stream));
-    FusedDecode fd{&DL, &ws};
+    const DecodeSink dec = decode_sink(DL, ws.counts, ws.n_hot, ws.hot, HotBuckets{});
     rc = loss_impl(scales, n_scales, loss_out, terms_out, nullptr, 0.5, loss_workspace, loss_workspace_bytes,
-                   stream_, &fd);
+                   stream_, &dec);
     if (rc != YB_OK || count_only) return rc;
     return decode_finish(DL, ws, false, rows, row_capacity, reinterpret_cast<long long*>(row_offsets), stream, true);
 }
@@ -1119,28 +1044,10 @@ static int step_impl(const yb_loss_scale* scales, int n_scales, float* loss_out,
     if (out_capacity < 0) return YB_E_CAPACITY;
     if (iou_mode != 1 && iou_mode != 2) return YB_E_PARAM;
     yb_decode_params dp;
-    memset(&dp, 0, sizeof(dp));
-    dp.version = scales[0].p.version;
-    dp.class_num = scales[0].p.class_num;
-    dp.n_scales = n_scales;
-    dp.is_f64 = 0;
-    dp.threshold = decode_threshold;
     const void* preds[YB_MAX_SCALES];
-    int64_t n_img = -1;
-    for (int s = 0; s < n_scales; ++s) {
-        const yb_loss_params& p = scales[s].p;
-        if (p.grid_h <= 0 || p.grid_w <= 0) return YB_E_SHAPE;
-        const int64_t cells = (int64_t)p.grid_h * p.grid_w;
-        if (scales[s].n_cells % cells != 0) return YB_E_SHAPE;
-        const int64_t n = scales[s].n_cells / cells;
-        if (n_img >= 0 && n != n_img) return YB_E_SHAPE;  // every scale must hold the same images
-        n_img = n;
-        if (p.class_num != dp.class_num || p.version != dp.version) return YB_E_PARAM;
-        dp.grid_h[s] = p.grid_h;
-        dp.grid_w[s] = p.grid_w;
-        dp.bbox_num[s] = p.bbox_num;
-        preds[s] = scales[s].y_pred;
-    }
+    int64_t n_img;
+    int rc = loss_decode_params(scales, n_scales, decode_threshold, dp, preds, n_img);
+    if (rc != YB_OK) return rc;
     if (n_img == 0) {
         if (!count_only) YB_CUDA_TRY(cudaMemsetAsync(out_offsets, 0, sizeof(int64_t), stream));
         if (n_overflow != nullptr) YB_CUDA_TRY(cudaMemsetAsync(n_overflow, 0, sizeof(unsigned int), stream));
@@ -1148,14 +1055,13 @@ static int step_impl(const yb_loss_scale* scales, int n_scales, float* loss_out,
                          stream_);
     }
     DecodeLaunch DL;
-    DecodeWs ws;
-    memset(&ws, 0, sizeof(ws));
-    int rc = fused_prepare(preds, n_img, &dp, rows_per_img_cap, fused_workspace, fused_workspace_bytes, DL, ws.buckets,
-                           stream, !clean);
+    HotBuckets K;
+    rc = fused_prepare(preds, n_img, &dp, rows_per_img_cap, fused_workspace, fused_workspace_bytes, DL, K, stream,
+                       !clean);
     if (rc != YB_OK) return rc;
-    FusedDecode fd{&DL, &ws};   // counts / flat list stay null: only the per-image buckets are filled
+    const DecodeSink dec = decode_sink(DL, nullptr, nullptr, nullptr, K);   // only the per-image buckets are filled
     rc = loss_impl(scales, n_scales, loss_out, terms_out, nullptr, 0.5, loss_workspace, loss_workspace_bytes, stream_,
-                   &fd, clean);
+                   &dec, clean);
     if (rc != YB_OK || count_only) return rc;
     return fused_finish(DL, n_img, rows_per_img_cap, fused_workspace, nms_threshold, iou_mode, out_rows, out_capacity,
                         out_offsets, n_overflow, stream);

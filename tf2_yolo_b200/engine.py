@@ -103,6 +103,66 @@ def make_loss_params(version, grid_shape, bbox_num, class_num, anchors=None, bin
     return p
 
 
+def floats_per_cell(p):
+    """Floats of one y_pred cell: v1 heads share one row of class scores between the boxes of a cell."""
+    return (5 * p.bbox_num + p.class_num) if p.version == 1 else p.bbox_num * (5 + p.class_num)
+
+
+def bind_loss_scales(params, y_trues, y_preds, global_batch=None, dpreds=None, want_grad=True, same_images=True,
+                     images=None):
+    """The yb_loss_scale array of one launch over the scales in ``params``.
+
+    y_trues[i]: (N, gh, gw, 5+C) fp32 CUDA; y_preds[i]: (N, gh, gw, info) fp32 CUDA.  ``same_images``:
+    every scale holds the N = y_preds[0].shape[0] images the decoding entry points need; without it each
+    scale's N follows from its own size.  ``images=(a, b)`` binds images a..b-1 of every tensor.
+    ``global_batch`` = divisor of reduce_mean(axis=0) (defaults to the scale's N).  The gradient goes to
+    ``dpreds`` (fresh tensors when None).  Returns (scales, dpreds list or None, number of images bound).
+    """
+    n = len(params)
+    if not (1 <= n <= N.YB_MAX_SCALES) or len(y_trues) != n or len(y_preds) != n:
+        raise ValueError("between 1 and 4 scales, one y_true / y_pred each")
+    require_cuda(*y_trues, *y_preds)
+    n_img = y_preds[0].shape[0]
+    a, b = images if images is not None else (0, None)
+    scales = (N.LossScale * n)()
+    outs = []
+    for i, (p, yt, yp) in enumerate(zip(params, y_trues, y_preds)):
+        if yt.dtype != torch.float32 or yp.dtype != torch.float32:
+            raise N.YoloB200Error("loss tensors must be float32 (Keras casts y_true to y_pred.dtype)")
+        cells_per_img, pcf, tcf = p.grid_h * p.grid_w, floats_per_cell(p), 5 + p.class_num
+        if yp.numel() % (cells_per_img * pcf) != 0:
+            raise ValueError(f"y_pred with {yp.numel()} elements does not reshape to (-1,{p.grid_h},{p.grid_w},{pcf})")
+        m = yp.numel() // (cells_per_img * pcf)
+        if yt.numel() != m * cells_per_img * tcf:
+            raise ValueError(f"y_true with {yt.numel()} elements does not reshape to ({m},{p.grid_h},{p.grid_w},{tcf})")
+        if same_images and m != n_img:
+            raise ValueError("every scale must hold the same images")
+        q = N.LossParams.from_buffer_copy(p)
+        q.inv_batch = 1.0 / float(global_batch if global_batch is not None else max(m, 1))
+        d = None
+        if want_grad:
+            d = dpreds[i] if dpreds is not None else torch.empty_like(yp)
+            require_cuda(d)
+        outs.append(d)
+        scales[i].y_true = yt.data_ptr() + 4 * a * cells_per_img * tcf
+        scales[i].y_pred = yp.data_ptr() + 4 * a * cells_per_img * pcf
+        scales[i].dpred = d.data_ptr() + 4 * a * cells_per_img * pcf if d is not None else None
+        scales[i].n_cells = ((b if b is not None else m) - a) * cells_per_img
+        scales[i].p = q
+    return scales, (outs if want_grad else None), (b - a if images is not None else n_img)
+
+
+def loss_decode_params(params, threshold):
+    """DecodeParams of the float32 heads ``params`` describe: the decode that the loss entry points
+    with a counting pass derive from their scales (yb_loss_decode_fused, yb_loss_decode_nms_fused)."""
+    p = N.DecodeParams()
+    p.version, p.class_num, p.n_scales, p.is_f64 = params[0].version, params[0].class_num, len(params), 0
+    for i, q in enumerate(params):
+        p.grid_h[i], p.grid_w[i], p.bbox_num[i] = q.grid_h, q.grid_w, q.bbox_num
+    p.threshold = float(threshold)
+    return p
+
+
 def loss_fwd_bwd(params, y_trues, y_preds, global_batch=None, want_grad=True, want_terms=False,
                  dpreds=None, want_metrics=False, recall_iou_threshold=0.5):
     """One fused launch over the scales in ``params``.
@@ -112,35 +172,8 @@ def loss_fwd_bwd(params, y_trues, y_preds, global_batch=None, want_grad=True, wa
     ``global_batch`` = divisor of reduce_mean(axis=0) (defaults to the local N).
     """
     n = len(params)
-    if not (1 <= n <= N.YB_MAX_SCALES) or len(y_trues) != n or len(y_preds) != n:
-        raise ValueError("between 1 and 4 scales, one y_true / y_pred each")
-    require_cuda(*y_trues, *y_preds)
+    scales, outs, _ = bind_loss_scales(params, y_trues, y_preds, global_batch, dpreds, want_grad, same_images=False)
     dev = y_preds[0].device
-    scales = (N.LossScale * n)()
-    outs = []
-    for i, (p, yt, yp) in enumerate(zip(params, y_trues, y_preds)):
-        if yt.dtype != torch.float32 or yp.dtype != torch.float32:
-            raise N.YoloB200Error("loss tensors must be float32 (Keras casts y_true to y_pred.dtype)")
-        cells_per_img = p.grid_h * p.grid_w
-        pcf = (5 * p.bbox_num + p.class_num) if p.version == 1 else p.bbox_num * (5 + p.class_num)
-        tcf = 5 + p.class_num
-        if yp.numel() % (cells_per_img * pcf) != 0:
-            raise ValueError(f"y_pred with {yp.numel()} elements does not reshape to (-1,{p.grid_h},{p.grid_w},{pcf})")
-        n_img = yp.numel() // (cells_per_img * pcf)
-        if yt.numel() != n_img * cells_per_img * tcf:
-            raise ValueError(f"y_true with {yt.numel()} elements does not reshape to ({n_img},{p.grid_h},{p.grid_w},{tcf})")
-        q = N.LossParams.from_buffer_copy(p)
-        q.inv_batch = 1.0 / float(global_batch if global_batch is not None else max(n_img, 1))
-        d = None
-        if want_grad:
-            d = dpreds[i] if dpreds is not None else torch.empty_like(yp)
-            require_cuda(d)
-        outs.append(d)
-        scales[i].y_true = yt.data_ptr()
-        scales[i].y_pred = yp.data_ptr()
-        scales[i].dpred = d.data_ptr() if d is not None else None
-        scales[i].n_cells = n_img * cells_per_img
-        scales[i].p = q
     with torch.cuda.device(dev):
         loss = torch.empty(n, dtype=torch.float32, device=dev)
         terms = torch.empty((n, N.YB_LOSS_TERMS), dtype=_F64, device=dev) if want_terms else None
@@ -151,10 +184,10 @@ def loss_fwd_bwd(params, y_trues, y_preds, global_batch=None, want_grad=True, wa
             N.check(N.lib.yb_loss_fwd_bwd_metrics(scales, n, _ptr(loss), _ptr(terms), _ptr(metrics),
                                                   float(recall_iou_threshold), _ptr(ws), ws_bytes, _stream()),
                     "yb_loss_fwd_bwd_metrics")
-            return loss, (outs if want_grad else None), terms, metrics
+            return loss, outs, terms, metrics
         N.check(N.lib.yb_loss_fwd_bwd(scales, n, _ptr(loss), _ptr(terms), _ptr(ws), ws_bytes, _stream()),
                 "yb_loss_fwd_bwd")
-    return loss, (outs if want_grad else None), terms
+    return loss, outs, terms
 
 
 def loss_decode_fused(params, y_trues, y_preds, threshold=0.5, global_batch=None, dpreds=None,
@@ -162,26 +195,9 @@ def loss_decode_fused(params, y_trues, y_preds, threshold=0.5, global_batch=None
     """Loss forward+gradient and decode of the same head outputs, y_pred read from HBM once
     (yb_loss_decode_fused).  Returns (loss [n], dpreds, terms, rows (capacity,7) f64, row_offsets)."""
     n = len(params)
-    require_cuda(*y_trues, *y_preds)
+    scales, outs, n_img = bind_loss_scales(params, y_trues, y_preds, global_batch, dpreds)
     dev = y_preds[0].device
-    scales = (N.LossScale * n)()
-    outs = []
-    n_img = y_preds[0].shape[0]
-    for i, (p, yt, yp) in enumerate(zip(params, y_trues, y_preds)):
-        if yt.dtype != torch.float32 or yp.dtype != torch.float32:
-            raise N.YoloB200Error("loss tensors must be float32")
-        cells_per_img = p.grid_h * p.grid_w
-        pcf = (5 * p.bbox_num + p.class_num) if p.version == 1 else p.bbox_num * (5 + p.class_num)
-        if yp.numel() != n_img * cells_per_img * pcf or yt.numel() != n_img * cells_per_img * (5 + p.class_num):
-            raise ValueError("every scale must hold the same images with matching grid / info sizes")
-        q = N.LossParams.from_buffer_copy(p)
-        q.inv_batch = 1.0 / float(global_batch if global_batch is not None else max(n_img, 1))
-        d = dpreds[i] if dpreds is not None else torch.empty_like(yp)
-        outs.append(d)
-        scales[i].y_true, scales[i].y_pred, scales[i].dpred = yt.data_ptr(), yp.data_ptr(), d.data_ptr()
-        scales[i].n_cells = n_img * cells_per_img
-        scales[i].p = q
-    dparams, _ = make_decode_params(y_preds, params[0].class_num, threshold, params[0].version)
+    dparams = loss_decode_params(params, threshold)
     if rows is not None:
         capacity = rows.shape[0]
     if capacity is None:
@@ -367,29 +383,6 @@ def decode_nms_batch_exact(preds, class_num=1, threshold=0.5, version=1, nms_thr
     return g["out_rows"][:int(g["out_offsets"][-1].item())], g["out_offsets"]
 
 
-def _fill_step_scales(params, y_trues, y_preds, global_batch, dpreds):
-    """yb_loss_scale array of a step over whole images (every scale holds the same n_img images)."""
-    n = len(params)
-    n_img = y_preds[0].shape[0]
-    scales = (N.LossScale * n)()
-    outs = []
-    for i, (p, yt, yp) in enumerate(zip(params, y_trues, y_preds)):
-        if yt.dtype != torch.float32 or yp.dtype != torch.float32:
-            raise N.YoloB200Error("loss tensors must be float32")
-        cells_per_img = p.grid_h * p.grid_w
-        pcf = (5 * p.bbox_num + p.class_num) if p.version == 1 else p.bbox_num * (5 + p.class_num)
-        if yp.numel() != n_img * cells_per_img * pcf or yt.numel() != n_img * cells_per_img * (5 + p.class_num):
-            raise ValueError("every scale must hold the same images with matching grid / info sizes")
-        q = N.LossParams.from_buffer_copy(p)
-        q.inv_batch = 1.0 / float(global_batch if global_batch is not None else max(n_img, 1))
-        d = dpreds[i] if dpreds is not None else torch.empty_like(yp)
-        outs.append(d)
-        scales[i].y_true, scales[i].y_pred, scales[i].dpred = yt.data_ptr(), yp.data_ptr(), d.data_ptr()
-        scales[i].n_cells = n_img * cells_per_img
-        scales[i].p = q
-    return scales, outs, n_img
-
-
 def loss_decode_nms_fused(params, y_trues, y_preds, threshold=0.5, nms_threshold=0.45, iou_mode=1,
                           rows_per_img_cap=1024, global_batch=None, dpreds=None, want_terms=False, out=None,
                           out_capacity=None, split_hook=None, loss_out=None, loss_box=None):
@@ -397,10 +390,9 @@ def loss_decode_nms_fused(params, y_trues, y_preds, threshold=0.5, nms_threshold
     gradient with the decode counting pass riding on its read of y_pred, then decode + NMS with one
     CTA per image.  Returns (loss [n], dpreds, terms, dict(out_rows, out_offsets, n_overflow))."""
     n = len(params)
-    require_cuda(*y_trues, *y_preds)
+    scales, outs, n_img = bind_loss_scales(params, y_trues, y_preds, global_batch, dpreds)
     dev = y_preds[0].device
-    scales, outs, n_img = _fill_step_scales(params, y_trues, y_preds, global_batch, dpreds)
-    dparams, _ = make_decode_params(y_preds, params[0].class_num, threshold, params[0].version)
+    dparams = loss_decode_params(params, threshold)
     if out_capacity is None:
         out_capacity = rows_per_img_cap * max(n_img, 1)
     with torch.cuda.device(dev):
@@ -452,13 +444,12 @@ class TrainEvalStep:
                  rows_per_img_cap=1024, global_batch=None, dpreds=None, want_terms=False, out=None,
                  out_capacity=None, tail=None, graph=True):
         n = len(params)
-        require_cuda(*y_trues, *y_preds)
+        self.scales, self.dpreds, n_img = bind_loss_scales(params, y_trues, y_preds, global_batch, dpreds)
         self.dev = dev = y_preds[0].device
         self.n = n
-        self.n_img = n_img = y_preds[0].shape[0]
+        self.n_img = n_img
         self._keep = (list(y_trues), list(y_preds))
-        self.scales, self.dpreds, _ = _fill_step_scales(params, y_trues, y_preds, global_batch, dpreds)
-        dparams, _ = make_decode_params(y_preds, params[0].class_num, threshold, params[0].version)
+        dparams = loss_decode_params(params, threshold)
         self.args = (float(threshold), float(nms_threshold), int(iou_mode), int(rows_per_img_cap))
         if out_capacity is None:
             out_capacity = rows_per_img_cap * max(n_img, 1)

@@ -69,11 +69,9 @@ class HostBatchStep:
         with torch.cuda.device(dev):
             self.copy_stream = torch.cuda.Stream(dev)
             self.compute_stream = torch.cuda.Stream(dev)
-            self.info = [(5 * p.bbox_num + p.class_num) if p.version == 1 else p.bbox_num * (5 + p.class_num)
-                         for p in self.params]
             f32 = torch.float32
-            self.y_pred = [torch.empty((self.batch, p.grid_h, p.grid_w, k), dtype=f32, device=dev)
-                           for p, k in zip(self.params, self.info)]
+            self.y_pred = [torch.empty((self.batch, p.grid_h, p.grid_w, engine.floats_per_cell(p)), dtype=f32,
+                                       device=dev) for p in self.params]
             self.dpred = [torch.empty_like(t) for t in self.y_pred]
             self.y_true = [torch.empty((self.batch, p.grid_h, p.grid_w, 5 + self.C), dtype=f32, device=dev)
                            for p in self.params]
@@ -88,10 +86,10 @@ class HostBatchStep:
             self.row_offsets = torch.empty(most + 1, dtype=torch.int64, device=dev)
             self.keep = torch.empty(cap, dtype=torch.uint8, device=dev)
             lws = N.lib.yb_loss_workspace_bytes(self.n_scales)
-            dp = self._decode_params(most)
-            dws = N.lib.yb_decode_workspace_bytes(C.byref(dp), most)
+            self.dparams = engine.loss_decode_params(self.params, self.thr)
+            dws = N.lib.yb_decode_workspace_bytes(C.byref(self.dparams), most)
             nws = N.lib.yb_nms_workspace_bytes(cap, most, self.C)
-            fws = N.lib.yb_decode_nms_workspace_bytes(C.byref(dp), most, self.rows_per_img)
+            fws = N.lib.yb_decode_nms_workspace_bytes(C.byref(self.dparams), most, self.rows_per_img)
             if fws == 0:
                 raise ValueError(f"rows_per_img must be in [32, {N.YB_FUSED_MAX_ROWS}] and class_num <= 256")
             self.ws = [torch.empty(int(b) + 256, dtype=torch.uint8, device=dev) for b in (lws, dws, nws, fws)]
@@ -107,32 +105,14 @@ class HostBatchStep:
         self.launches_per_step = 3 * nc   # encode, loss + count, decode + NMS
 
     # -- argument binding (once) ---------------------------------------------------------------
-    def _decode_params(self, n_img):
-        p = N.DecodeParams()
-        p.version, p.class_num, p.n_scales, p.is_f64 = self.version, self.C, self.n_scales, 0
-        for i, q in enumerate(self.params):
-            p.grid_h[i], p.grid_w[i], p.bbox_num[i] = q.grid_h, q.grid_w, q.bbox_num
-        p.threshold = self.thr
-        return p
-
     @staticmethod
     def _al(t):
         return t.data_ptr() + ((-t.data_ptr()) % 256)
 
     def _bind_chunk(self, ci, a, b):
-        n = b - a
-        scales = (N.LossScale * self.n_scales)()
-        label_ptrs = (C.c_void_p * self.n_scales)()
-        for s, p in enumerate(self.params):
-            cells = p.grid_h * p.grid_w
-            q = N.LossParams.from_buffer_copy(p)
-            q.inv_batch = 1.0 / float(self.global_batch)
-            scales[s].y_true = self.y_true[s].data_ptr() + 4 * a * cells * (5 + self.C)
-            scales[s].y_pred = self.y_pred[s].data_ptr() + 4 * a * cells * self.info[s]
-            scales[s].dpred = self.dpred[s].data_ptr() + 4 * a * cells * self.info[s]
-            scales[s].n_cells = n * cells
-            scales[s].p = q
-            label_ptrs[s] = scales[s].y_true
+        scales, _, n = engine.bind_loss_scales(self.params, self.y_true, self.y_pred, self.global_batch, self.dpred,
+                                               images=(a, b))
+        label_ptrs = (C.c_void_p * self.n_scales)(*[scales[s].y_true for s in range(self.n_scales)])
         vp = C.c_void_p
         lws, dws, nws, fws = (vp(self._al(w)) for w in self.ws)
         pred_ptrs = (C.c_void_p * self.n_scales)(*[scales[s].y_pred for s in range(self.n_scales)])
@@ -204,14 +184,13 @@ class HostBatchStep:
         """Decode + NMS of one chunk with the general chain (any number of rows per image)."""
         lib, vp = N.lib, C.c_void_p
         n = call["n"]
-        dp = self._decode_params(n)
         cap = self.row_cap
         while True:
             rows = torch.empty((cap, 7), dtype=torch.float64, device=self.dev)
             roff = torch.empty(n + 1, dtype=torch.int64, device=self.dev)
             keep = torch.empty(cap, dtype=torch.uint8, device=self.dev)
-            N.check(lib.yb_decode(call["pred_ptrs"], n, C.byref(dp), vp(rows.data_ptr()), cap, vp(roff.data_ptr()),
-                                  call["dws"], self.ws_bytes[1], k), "yb_decode")
+            N.check(lib.yb_decode(call["pred_ptrs"], n, C.byref(self.dparams), vp(rows.data_ptr()), cap,
+                                  vp(roff.data_ptr()), call["dws"], self.ws_bytes[1], k), "yb_decode")
             self.compute_stream.synchronize()
             total = int(roff[-1].item())
             if total <= cap:

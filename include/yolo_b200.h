@@ -128,6 +128,14 @@ int yb_loss_v4_fwd_bwd(const float* y_true, const float* y_pred, int64_t n_cells
                        float* loss_out, float* dpred, const yb_loss_params* p,
                        void* workspace, size_t workspace_bytes, yb_stream_t stream);
 
+/* The head transform of yolov4/models/__init__.py:42-60 (yolov3/models/__init__.py:36-63) on raw head
+ * outputs, v3/v4 layout (B*(5+C) floats per cell): sigmoid x, y, objectness and class scores,
+ * anchor * exp for w, h - the same float32 arithmetic the loss kernel applies with from_logits, so
+ * decoding the result gives the rows the two-launch step gives for the raw heads.
+ * p: the scale's loss parameters (version 3|4, has_anchors, bbox_num, class_num, anchors are read).
+ * out may alias raw (out == raw: in place). */
+int yb_activate_head(const yb_loss_params* p, const float* raw, float* out, int64_t n_cells, yb_stream_t stream);
+
 /* Grid IoU (and CIoU) of the label box of a cell against its B predicted boxes:
  * yolov4/losses/loss.py:10-61 (cal_iou); v1-v3 loss.py:9-37.  box_true is
  * (n_cells, true_stride) with xywh at [0:4]; box_pred (n_cells, B, pred_stride).
@@ -169,7 +177,8 @@ int yb_decode(const void* const* preds_host /* n_scales device pointers */,
  * tiles the loss kernel already staged in shared memory; only cells with hits are touched again
  * to emit rows.  Results are identical to calling the two entry points separately.
  * With row_offsets == NULL only the counting pass runs (the counts stay in decode_workspace);
- * yb_decode_finish then scans them and emits the rows. */
+ * yb_decode_finish then scans them and emits the rows.  The rows are read back from y_pred, so
+ * from_logits scales are rejected (YB_E_PARAM): activate raw heads with yb_activate_head first. */
 int yb_loss_decode_fused(const yb_loss_scale* scales_host, int n_scales, float* loss_out,
                          double* terms_out, double decode_threshold, double* rows,
                          int64_t row_capacity, int64_t* row_offsets, void* loss_workspace,
@@ -225,6 +234,10 @@ int yb_soft_nms(const double* rows, const int64_t* row_offsets, int64_t n_rows, 
  * forward + gradient (as yb_loss_fwd_bwd) with the counting pass riding on its read of y_pred,
  * then the per-image kernel.  With out_offsets == NULL only the loss kernel runs (the buckets
  * stay in fused_workspace); yb_decode_nms_finish then launches the per-image kernel.
+ * The step also takes RAW v3/v4 heads (from_logits on every scale): the counting pass applies the
+ * head transform of yb_activate_head to the values it files, so the survivors are those of the
+ * activated heads, and the gradient is d/d(raw).  The overflow fallback then decodes the
+ * yb_activate_head output, not the raw heads.
  * ---------------------------------------------------------------------- */
 size_t yb_decode_nms_workspace_bytes(const yb_decode_params* p, int64_t n_img, int rows_per_img_cap);
 

@@ -84,6 +84,7 @@ SIGNATURES = {
     "yb_loss_v2_fwd_bwd": (C.c_int, [_vp, _vp, _i64, _vp, _vp, C.POINTER(LossParams), _vp, _sz, _vp]),
     "yb_loss_v3_fwd_bwd": (C.c_int, [_vp, _vp, _i64, _vp, _vp, C.POINTER(LossParams), _vp, _sz, _vp]),
     "yb_loss_v4_fwd_bwd": (C.c_int, [_vp, _vp, _i64, _vp, _vp, C.POINTER(LossParams), _vp, _sz, _vp]),
+    "yb_activate_head": (C.c_int, [C.POINTER(LossParams), _vp, _vp, _i64, _vp]),
     "yb_grid_iou": (C.c_int, [_vp, _i32, _vp, _i32, _i64, _i32, _i32, _i32, _vp, _vp, _vp]),
     "yb_decode_workspace_bytes": (_sz, [C.POINTER(DecodeParams), _i64]),
     "yb_decode": (C.c_int, [C.POINTER(_vp), _i64, C.POINTER(DecodeParams), _vp, _i64, _vp, _vp, _sz, _vp]),

@@ -2,6 +2,7 @@
 // loss+decode launch in loss.cu.
 #pragma once
 #include "common.cuh"
+#include "head_transform.cuh"
 
 namespace yb {
 
@@ -87,18 +88,13 @@ struct LaneHits {
     unsigned base;     // first of the n slots reserved in the image's bucket
 };
 
-// Counting pass of one lane = one box (lane = cell*B + box, B lanes per cell) of cell g of scale s:
-// hits of c*p_k >= thr over the box's C class scores `prob`, the cell's count (by shuffle, lane of box
-// 0) and the box's work-list entry where those sinks are set, and the reservation of the box's rows
-// in its image's bucket.  Called by whole warps; `valid` = the lane holds a box.
-template <typename T>
-__device__ __forceinline__ LaneHits decode_count_lane(const DecodeSink& K, bool valid, const T* prob, T c, T thr,
-                                                      int C, int B, int lc, int lb, int s, long long g) {
-    LaneHits h = {0, 0u, 0u, 0u, 0u};
-    if (valid) {
-#pragma unroll 16
-        for (int k = 0; k < C; ++k) h.n += (mul_rn<T>(c, prob[k]) >= thr) ? 1 : 0;
-    }
+// What the counting pass does with the n hits of one lane = one box (lane = cell*B + box, B lanes per
+// cell) of cell g of scale s: the cell's count (by shuffle, lane of box 0) and the box's work-list entry
+// where those sinks are set, and the reservation of the box's rows in its image's bucket.  Called by
+// whole warps; `valid` = the lane holds a box.
+__device__ __forceinline__ LaneHits decode_place_lane(const DecodeSink& K, bool valid, int n, int B, int lc, int lb,
+                                                      int s, long long g) {
+    LaneHits h = {n, 0u, 0u, 0u, 0u};
     int tot = 0, before = 0;
     for (int q = 0; q < B; ++q) {
         const int nq = __shfl_sync(0xffffffffu, h.n, lc * B + q);
@@ -121,11 +117,50 @@ __device__ __forceinline__ LaneHits decode_count_lane(const DecodeSink& K, bool 
     return h;
 }
 
+// Counting pass of one lane: hits of c*p_k >= thr over the box's C class scores `prob`, then
+// decode_place_lane.
+template <typename T>
+__device__ __forceinline__ LaneHits decode_count_lane(const DecodeSink& K, bool valid, const T* prob, T c, T thr,
+                                                      int C, int B, int lc, int lb, int s, long long g) {
+    int n = 0;
+    if (valid) {
+#pragma unroll 16
+        for (int k = 0; k < C; ++k) n += (mul_rn<T>(c, prob[k]) >= thr) ? 1 : 0;
+    }
+    return decode_place_lane(K, valid, n, B, lc, lb, s, g);
+}
+
+// Hits of c*sigmoidf_(p_k) >= thr of the warp's boxes whose class scores are RAW logits (the from-logits
+// loss kernel; c is already activated).  A box with c < thr has none, exactly: sigmoidf_ <= 1, so
+// c*sigmoidf_(p) rounds to at most c, and a NaN product fails the >= test.  The few other boxes are
+// served by the whole WARP, one at a time, 32 scores per step: a lane walking its own C scores would
+// stall the other 31.  Returns the hits of the lane's own box; `prob_at` = offset of its scores in `tile`.
+__device__ __forceinline__ int decode_hits_logits(bool valid, const float* tile, int prob_at, float c, float thr,
+                                                  int C, int lane) {
+    int n = 0;
+    unsigned cand = __ballot_sync(0xffffffffu, valid && !(c < thr));
+    while (cand) {
+        const int src = __ffs(cand) - 1;
+        cand &= cand - 1;
+        const float* hprob = tile + __shfl_sync(0xffffffffu, prob_at, src);
+        const float hc = __shfl_sync(0xffffffffu, c, src);
+        int hits = 0;
+        for (int k0 = 0; k0 < C; k0 += 32) {
+            const int k = k0 + lane;
+            const bool hit = (k < C) && (mul_rn<float>(hc, sigmoidf_(hprob[k])) >= thr);
+            hits += __popc(__ballot_sync(0xffffffffu, hit));
+        }
+        if (lane == src) n = hits;
+    }
+    return n;
+}
+
 // The rows of the warp's boxes with hits into their images' buckets, the WARP serving one hot box at a
 // time (32 class scores per step, ballot, lane-parallel row writes): a lane walking its own C scores
 // again would stall the other 31 for C steps.  Each lane passes its box's values and the offset of its
-// class scores in `tile`; only the hot lanes' are read.
-template <typename T>
+// class scores in `tile`; only the hot lanes' are read.  kLogits: the scores are raw logits, the rows
+// get sigmoidf_(p_k) - the value decode_hits_logits counted.
+template <typename T, bool kLogits = false>
 __device__ __forceinline__ void decode_file_rows(const HotBuckets& K, const LaneHits& h, const T* tile, int prob_at,
                                                  int lb, T x, T y, T w, T hgt, T c, T thr, int C, int lane) {
     unsigned hot = __ballot_sync(0xffffffffu, h.n > 0);
@@ -144,7 +179,7 @@ __device__ __forceinline__ void decode_file_rows(const HotBuckets& K, const Lane
         FusedRow* dst = K.row + (size_t)himg * K.cap;
         for (int k0 = 0; k0 < C; k0 += 32) {
             const int k = k0 + lane;
-            const T p = (k < C) ? hprob[k] : (T)0;
+            const T p = (k < C) ? (kLogits ? sigmoidf_(hprob[k]) : hprob[k]) : (T)0;
             const bool hit = (k < C) && (mul_rn<T>(hc, p) >= thr);
             const unsigned m = __ballot_sync(0xffffffffu, hit);
             const unsigned at = u + __popc(m & ((1u << lane) - 1u));

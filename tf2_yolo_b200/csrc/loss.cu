@@ -257,8 +257,6 @@ __device__ __forceinline__ int warp_argmax(const float* v, int C, int lane) {
     return arg;
 }
 
-__device__ __forceinline__ float sigmoidf_(float z) { return 1.f / (1.f + expf(-z)); }
-
 #ifdef YB_LOSS_PROFILE
 __device__ unsigned long long yb_loss_prof[1024 * 6];
 __device__ __forceinline__ unsigned long long gtimer() {
@@ -446,8 +444,8 @@ loss_fwd_bwd_kernel(const __grid_constant__ LossLaunch L) {
                     px = pc[0]; py = pc[1]; pw = pc[2]; ph = pc[3]; c = pc[4];
                     tx = tc[0]; ty = tc[1]; tw = tc[2]; th = tc[3]; obj = tc[4];
                     if (kLogits) {  // head transform: sigmoid offsets / objectness, anchor * exp sizes
-                        px = sigmoidf_(px); py = sigmoidf_(py); c = sigmoidf_(c);
-                        pw = aw * expf(pw); ph = ah * expf(ph);
+                        px = head_act(px, 0, aw); py = head_act(py, 1, ah); c = head_act(c, 4, aw);
+                        pw = head_act(pw, 2, aw); ph = head_act(ph, 3, ah);
                     }
                 }
                 const float iou = grid_iou_f32(px, py, pw, ph, tx, ty, tw, th, S.gw, S.gh);
@@ -467,8 +465,13 @@ loss_fwd_bwd_kernel(const __grid_constant__ LossLaunch L) {
                 // filed after the loss arithmetic below, which hides the atomic's round trip to L2.
                 // Both must precede the in-place gradient writes.
                 const int prob_at = cell * S.pcf + ((V == 1) ? 5 * B : lb * bstride + 5);   // the box's class scores
+                // Raw-logit heads: the scores are activated on the fly (c already is), the warp serving the
+                // few boxes that pass the exact prefilter c >= thr.
                 LaneHits dec = {0, 0u, 0u, 0u, 0u};
-                if (kDecode)
+                if constexpr (kDecode && kLogits)
+                    dec = decode_place_lane(L.dec, valid, decode_hits_logits(valid, sp, prob_at, c, L.dec.thr, C, lane),
+                                            B, lc, lb, s, cell0 + cell);
+                else if (kDecode)
                     dec = decode_count_lane<float>(L.dec, valid, sp + prob_at, c, L.dec.thr, C, B, lc, lb, s,
                                                    cell0 + cell);
                 if (kMetrics) {
@@ -621,7 +624,8 @@ loss_fwd_bwd_kernel(const __grid_constant__ LossLaunch L) {
                     }
                 }
                 if (kDecode && L.dec.buckets.n != nullptr)   // before the gradients overwrite the tile
-                    decode_file_rows<float>(L.dec.buckets, dec, sp, prob_at, lb, px, py, pw, ph, c, L.dec.thr, C, lane);
+                    decode_file_rows<float, kLogits>(L.dec.buckets, dec, sp, prob_at, lb, px, py, pw, ph, c, L.dec.thr, C,
+                                                     lane);
                 if (valid) {
                     if (write) {
                         pc[0] = g0; pc[1] = g1; pc[2] = g2; pc[3] = g3; pc[4] = g4;
@@ -736,6 +740,64 @@ __global__ void grid_iou_kernel(const float* __restrict__ bt, int ts, const floa
     }
 }
 
+// ---- head transform of raw heads (yb_activate_head) ----------------------------
+// Elementwise over the flattened (n_cells, B, 5+C) head, kW floats per access (4: 16-byte aligned
+// tensors).  A thread keeps the (box, value) position of its first float and advances it by the
+// grid stride (adv_b boxes + adv_j values) instead of dividing per element.  out may alias raw.
+struct HeadAnchors {
+    float a[2 * YB_MAX_BOXES];
+};
+
+template <int kW>
+__global__ void __launch_bounds__(256) activate_head_kernel(const float* raw, float* out, long long n_items,
+                                                            int n_tail, int bs, int B, int adv_b, int adv_j,
+                                                            const __grid_constant__ HeadAnchors anc) {
+    __shared__ float s_anc[2 * YB_MAX_BOXES];
+    if (threadIdx.x < 2 * YB_MAX_BOXES) s_anc[threadIdx.x] = anc.a[threadIdx.x];
+    __syncthreads();
+    const long long cell_floats = (long long)B * bs;
+    const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const int r = (int)((i0 * kW) % cell_floats);
+    int b = r / bs, j = r - b * bs;
+    for (long long i = i0; i < n_items; i += stride) {
+        float v[kW];
+        if constexpr (kW == 4) {
+            const float4 q = reinterpret_cast<const float4*>(raw)[i];
+            v[0] = q.x; v[1] = q.y; v[2] = q.z; v[3] = q.w;
+        } else {
+            v[0] = raw[i];
+        }
+#pragma unroll
+        for (int t = 0; t < kW; ++t) {
+            int jt = j + t, bt = b;
+            if (jt >= bs) {   // bs = 5 + C > 4: at most one box boundary inside an access
+                jt -= bs;
+                if (++bt == B) bt = 0;
+            }
+            v[t] = head_act(v[t], jt, s_anc[2 * bt + (jt == 3 ? 1 : 0)]);
+        }
+        if constexpr (kW == 4) {
+            reinterpret_cast<float4*>(out)[i] = make_float4(v[0], v[1], v[2], v[3]);
+        } else {
+            out[i] = v[0];
+        }
+        j += adv_j;
+        b += adv_b;
+        if (j >= bs) {
+            j -= bs;
+            ++b;
+        }
+        if (b >= B) b -= B;
+    }
+    // the n_tail (< kW) floats after the last full access
+    if (blockIdx.x == 0 && (int)threadIdx.x < n_tail) {
+        const long long e = n_items * kW + threadIdx.x;
+        const int re = (int)(e % cell_floats), be = re / bs, je = re - be * bs;
+        out[e] = head_act(raw[e], je, s_anc[2 * be + (je == 3 ? 1 : 0)]);
+    }
+}
+
 // ---- host side ----------------------------------------------------------------
 
 // Tuning knobs (YB_LOSS_STAGES, YB_LOSS_CTAS_PER_SM, YB_LOSS_TILE_CELLS, YB_LOSS_WARPS): read from the environment
@@ -814,25 +876,29 @@ static int launch_loss_variant(const LossLaunch& L, int grid, int threads, size_
     return YB_OK;
 }
 
-template <int V, bool kMetrics>
+template <int V, bool kMetrics, bool kDecode>
 static int launch_loss_logits(const LossLaunch& L, int grid, int threads, size_t smem, cudaStream_t stream) {
     static SmemRaised done;
-    YB_CUDA_TRY(raise_dynamic_smem_once(loss_fwd_bwd_kernel<V, kMetrics, false, true>, (int)smem, &done));
-    loss_fwd_bwd_kernel<V, kMetrics, false, true><<<grid, threads, smem, stream>>>(L);
+    YB_CUDA_TRY(raise_dynamic_smem_once(loss_fwd_bwd_kernel<V, kMetrics, kDecode, true>, (int)smem, &done));
+    loss_fwd_bwd_kernel<V, kMetrics, kDecode, true><<<grid, threads, smem, stream>>>(L);
     YB_CUDA_TRY(cudaGetLastError());
     return YB_OK;
 }
 
+// d: the launch carries a counting pass.  From logits, that is only the per-image buckets of the
+// two-launch step (step_impl): the other counting passes are followed by an emit pass that re-reads
+// the head tensors (yb_loss_decode_fused rejects raw heads before it gets here), and metrics do not
+// ride on the step.
 template <int V>
 static int launch_loss(const LossLaunch& L, bool d, int grid, int threads, size_t smem, cudaStream_t stream) {
     const bool m = L.metrics_out != nullptr;
     if (L.from_logits) {
         if (V != 3 && V != 4) return YB_E_PARAM;  // v1/v2 heads end in a softmax
-        if (d) return YB_E_PARAM;                 // decode counting needs activated scores
         if (V == 3 || V == 4) {
             constexpr int W = (V == 3 || V == 4) ? V : 4;
-            return m ? launch_loss_logits<W, true>(L, grid, threads, smem, stream)
-                     : launch_loss_logits<W, false>(L, grid, threads, smem, stream);
+            if (d) return launch_loss_logits<W, false, true>(L, grid, threads, smem, stream);
+            return m ? launch_loss_logits<W, true, false>(L, grid, threads, smem, stream)
+                     : launch_loss_logits<W, false, false>(L, grid, threads, smem, stream);
         }
     }
     if (m && d) return launch_loss_variant<V, true, true>(L, grid, threads, smem, stream);
@@ -980,6 +1046,9 @@ static int loss_decode_params(const yb_loss_scale* scales, int n_scales, double 
     n_img = -1;
     for (int s = 0; s < n_scales; ++s) {
         const yb_loss_params& p = scales[s].p;
+        // raw heads: every scale, and only the sigmoid heads of v3/v4 (v1/v2 end in a softmax)
+        if ((p.from_logits != 0) != (scales[0].p.from_logits != 0)) return YB_E_PARAM;
+        if (p.from_logits && p.version != 3 && p.version != 4) return YB_E_PARAM;
         if (p.grid_h <= 0 || p.grid_w <= 0) return YB_E_SHAPE;
         const int64_t cells = (int64_t)p.grid_h * p.grid_w;
         if (scales[s].n_cells % cells != 0) return YB_E_SHAPE;
@@ -1007,6 +1076,10 @@ extern "C" int yb_loss_decode_fused(const yb_loss_scale* scales, int n_scales, f
     if (rows == nullptr && row_capacity > 0) return YB_E_NULL;
     const bool count_only = row_offsets == nullptr;  // rows are emitted later by yb_decode_finish
     if (row_capacity < 0) return YB_E_CAPACITY;
+    // the emit pass reads the rows back from the head tensors, which must hold activated values:
+    // activate raw heads with yb_activate_head first
+    for (int s = 0; s < n_scales; ++s)
+        if (scales[s].p.from_logits) return YB_E_PARAM;
     yb_decode_params dp;
     const void* preds[YB_MAX_SCALES];
     int64_t n_img;
@@ -1120,6 +1193,35 @@ YB_DEFINE_LOSS(1)
 YB_DEFINE_LOSS(2)
 YB_DEFINE_LOSS(3)
 YB_DEFINE_LOSS(4)
+
+extern "C" int yb_activate_head(const yb_loss_params* p, const float* raw, float* out, int64_t n_cells,
+                                yb_stream_t stream_) {
+    cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+    if (p == nullptr || raw == nullptr || out == nullptr) return YB_E_NULL;
+    if ((p->version != 3 && p->version != 4) || !p->has_anchors) return YB_E_PARAM;
+    if (p->bbox_num <= 0 || p->bbox_num > YB_MAX_BOXES || p->class_num <= 0 || n_cells < 0) return YB_E_SHAPE;
+    const long long bs = 5LL + p->class_num, cell_floats = p->bbox_num * bs;
+    if (n_cells > INT64_MAX / cell_floats || cell_floats > INT32_MAX) return YB_E_SHAPE;
+    if (((uintptr_t)raw | (uintptr_t)out) & 3) return YB_E_ALIGN;
+    const long long n = n_cells * cell_floats;
+    if (n == 0) return YB_OK;
+    HeadAnchors anc;
+    for (int i = 0; i < 2 * YB_MAX_BOXES; ++i) anc.a[i] = (i < 2 * p->bbox_num) ? p->anchors[i] : 1.f;
+    const bool vec = (((uintptr_t)raw | (uintptr_t)out) & 15) == 0;
+    const int kw = vec ? 4 : 1, threads = 256;
+    const long long n_items = n / kw;
+    const int blocks = (int)max(1LL, min((long long)kNumSMs * 8, (n_items + threads - 1) / threads));
+    const long long adv = ((long long)blocks * threads * kw) % cell_floats;
+    const int adv_b = (int)(adv / bs), adv_j = (int)(adv % bs), n_tail = (int)(n - n_items * kw);
+    if (vec)
+        activate_head_kernel<4><<<blocks, threads, 0, stream>>>(raw, out, n_items, n_tail, (int)bs, p->bbox_num, adv_b,
+                                                                 adv_j, anc);
+    else
+        activate_head_kernel<1><<<blocks, threads, 0, stream>>>(raw, out, n_items, n_tail, (int)bs, p->bbox_num, adv_b,
+                                                                 adv_j, anc);
+    YB_CUDA_TRY(cudaGetLastError());
+    return YB_OK;
+}
 
 extern "C" int yb_grid_iou(const float* box_true, int true_stride, const float* box_pred,
                            int pred_stride, int64_t n_cells, int bbox_num, int grid_h, int grid_w,

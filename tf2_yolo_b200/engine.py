@@ -193,7 +193,9 @@ def loss_fwd_bwd(params, y_trues, y_preds, global_batch=None, want_grad=True, wa
 def loss_decode_fused(params, y_trues, y_preds, threshold=0.5, global_batch=None, dpreds=None,
                       capacity=None, rows=None, want_terms=False, split_hook=None):
     """Loss forward+gradient and decode of the same head outputs, y_pred read from HBM once
-    (yb_loss_decode_fused).  Returns (loss [n], dpreds, terms, rows (capacity,7) f64, row_offsets)."""
+    (yb_loss_decode_fused).  Returns (loss [n], dpreds, terms, rows (capacity,7) f64, row_offsets).
+    Activated heads only: the rows are read back from y_pred (raw heads: loss_decode_nms_fused, or
+    activate_head first)."""
     n = len(params)
     scales, outs, n_img = bind_loss_scales(params, y_trues, y_preds, global_batch, dpreds)
     dev = y_preds[0].device
@@ -225,6 +227,28 @@ def loss_decode_fused(params, y_trues, y_preds, threshold=0.5, global_batch=None
             N.check(N.lib.yb_decode_finish(ptrs, n_img, C.byref(dparams), _ptr(rows), capacity, _ptr(offsets),
                                            _ptr(dws), dws_bytes, _stream()), "yb_decode_finish")
     return loss, outs, terms, rows, offsets
+
+
+def activate_head(params, raw, out=None):
+    """The head transform of one v3/v4 scale on the device (yb_activate_head): sigmoid on x, y,
+    objectness and class scores, anchor * exp on w, h of the raw head outputs ``raw`` (N, gh, gw,
+    B*(5+C)) fp32 CUDA, with the anchors of ``params`` (the scale's LossParams).  The same float32
+    arithmetic as the from-logits loss kernel, so decoding the result gives the rows the two-launch
+    step gives for ``raw``.  ``out`` may be ``raw`` (in place).  Returns the activated tensor."""
+    require_cuda(raw, out)
+    if raw.dtype != torch.float32 or (out is not None and out.dtype != torch.float32):
+        raise N.YoloB200Error("activate_head: float32 heads")
+    pcf = floats_per_cell(params)
+    if raw.numel() % pcf != 0:
+        raise ValueError(f"a head of {raw.numel()} floats does not reshape to (-1, {pcf})")
+    if out is None:
+        out = torch.empty_like(raw)
+    elif out.numel() != raw.numel():
+        raise ValueError("out must have the size of raw")
+    with torch.cuda.device(raw.device):
+        N.check(N.lib.yb_activate_head(C.byref(params), _ptr(raw), _ptr(out), raw.numel() // pcf, _stream()),
+                "yb_activate_head")
+    return out
 
 
 def grid_iou(box_true, box_pred, grid_shape, want_ciou=False):
@@ -388,7 +412,11 @@ def loss_decode_nms_fused(params, y_trues, y_preds, threshold=0.5, nms_threshold
                           out_capacity=None, split_hook=None, loss_out=None, loss_box=None):
     """The train-and-evaluate step in two launches (yb_loss_decode_nms_fused): loss forward +
     gradient with the decode counting pass riding on its read of y_pred, then decode + NMS with one
-    CTA per image.  Returns (loss [n], dpreds, terms, dict(out_rows, out_offsets, n_overflow))."""
+    CTA per image.  Returns (loss [n], dpreds, terms, dict(out_rows, out_offsets, n_overflow)).
+    ``params`` with from_logits (grid_loss.wrap_yolo_loss_from_logits): y_preds hold the RAW v3/v4
+    head outputs, the gradient is d/d(raw) and the survivors are those of the activated heads
+    (activate_head).  An image over ``rows_per_img_cap`` rows has no survivors and is counted in
+    n_overflow: take it from decode_nms_batch_exact on the activated heads."""
     n = len(params)
     scales, outs, n_img = bind_loss_scales(params, y_trues, y_preds, global_batch, dpreds)
     dev = y_preds[0].device
@@ -438,13 +466,16 @@ class TrainEvalStep:
     once and replayed by run().  graph=False launches the same two kernels eagerly.
     A collective is better issued after run() than captured through `tail`: bench.py alternates two
     steps and all-reduces each one's loss asynchronously (a graph that holds NCCL kernels has to be
-    destroyed before the process group, or the teardown can hang)."""
+    destroyed before the process group, or the teardown can hang).
+    ``params`` may be from-logits params (raw v3/v4 heads, see loss_decode_nms_fused); a step that
+    reports n_overflow takes its survivors from fallback_survivors()."""
 
     def __init__(self, params, y_trues, y_preds, threshold=0.5, nms_threshold=0.45, iou_mode=1,
                  rows_per_img_cap=1024, global_batch=None, dpreds=None, want_terms=False, out=None,
                  out_capacity=None, tail=None, graph=True):
         n = len(params)
         self.scales, self.dpreds, n_img = bind_loss_scales(params, y_trues, y_preds, global_batch, dpreds)
+        self.params = [N.LossParams.from_buffer_copy(p) for p in params]
         self.dev = dev = y_preds[0].device
         self.n = n
         self.n_img = n_img
@@ -510,6 +541,19 @@ class TrainEvalStep:
                 self._launch()
         return self.loss, self.dpreds, self.terms, dict(out_rows=self.out_rows, out_offsets=self.out_offsets,
                                                         n_overflow=self.n_overflow)
+
+    def fallback_survivors(self):
+        """The survivors of the current inputs from the checked decode + NMS (decode_nms_batch_exact,
+        any number of rows per image): what a step that reported n_overflow > 0 falls back to.  Raw
+        heads (from-logits params) are activated first, into fresh tensors.  Returns (rows (K,7) f64,
+        offsets (n_img+1) i64), both CUDA."""
+        thr, nms_thr, mode, cap = self.args
+        p0 = self.params[0]
+        preds = self._keep[1]
+        if p0.from_logits:
+            preds = [activate_head(p, t) for p, t in zip(self.params, preds)]
+        with torch.cuda.device(self.dev):
+            return decode_nms_batch_exact(preds, p0.class_num, thr, p0.version, nms_thr, mode, cap)
 
 
 def pairwise_iou(a, b, mode=1):

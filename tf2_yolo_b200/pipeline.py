@@ -16,7 +16,9 @@ Per chunk (all through the C ABI, include/yolo_b200.h): yb_encode_labels ->
 yb_loss_decode_nms_fused (loss fwd+grad with the decode counting pass riding on its read of
 y_pred, then decode + NMS with one CTA per image): three launches.  A chunk in which an image
 exceeds ``rows_per_img`` decode rows is redone after the step's sync with the general chain
-(yb_decode + yb_nms).  Chunk losses are partial sums with the divisor of the whole (global) batch,
+(yb_decode + yb_nms); with raw-logit heads (loss functions of wrap_yolo_loss_from_logits) the chunk
+is first activated into a scratch buffer (yb_activate_head), since yb_decode reads activated heads.
+Chunk losses are partial sums with the divisor of the whole (global) batch,
 so their sum is the reference's ``reduce_mean(axis=0)`` loss (yolov4/losses/loss.py:117).
 """
 import ctypes as C
@@ -94,6 +96,9 @@ class HostBatchStep:
                 raise ValueError(f"rows_per_img must be in [32, {N.YB_FUSED_MAX_ROWS}] and class_num <= 256")
             self.ws = [torch.empty(int(b) + 256, dtype=torch.uint8, device=dev) for b in (lws, dws, nws, fws)]
             self.ws_bytes = (lws, dws, nws, fws)
+            # raw heads: the activated heads of one chunk, what the overflow fallback decodes
+            self.act = ([torch.empty((most, p.grid_h, p.grid_w, engine.floats_per_cell(p)), dtype=f32, device=dev)
+                         for p in self.params] if p0.from_logits else None)
         # results, written by the kernels into mapped pinned host memory
         nc = len(self.chunks)
         self.loss_host = torch.zeros((nc, self.n_scales), dtype=torch.float32).pin_memory()
@@ -185,11 +190,17 @@ class HostBatchStep:
         lib, vp = N.lib, C.c_void_p
         n = call["n"]
         cap = self.row_cap
+        pred_ptrs = call["pred_ptrs"]
+        if self.act is not None:
+            for s, (p, a) in enumerate(zip(self.params, self.act)):
+                N.check(lib.yb_activate_head(C.byref(p), vp(pred_ptrs[s]), vp(a.data_ptr()), n * p.grid_h * p.grid_w,
+                                             k), "yb_activate_head")
+            pred_ptrs = (C.c_void_p * self.n_scales)(*[a.data_ptr() for a in self.act])
         while True:
             rows = torch.empty((cap, 7), dtype=torch.float64, device=self.dev)
             roff = torch.empty(n + 1, dtype=torch.int64, device=self.dev)
             keep = torch.empty(cap, dtype=torch.uint8, device=self.dev)
-            N.check(lib.yb_decode(call["pred_ptrs"], n, C.byref(self.dparams), vp(rows.data_ptr()), cap,
+            N.check(lib.yb_decode(pred_ptrs, n, C.byref(self.dparams), vp(rows.data_ptr()), cap,
                                   vp(roff.data_ptr()), call["dws"], self.ws_bytes[1], k), "yb_decode")
             self.compute_stream.synchronize()
             total = int(roff[-1].item())
